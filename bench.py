@@ -2,7 +2,7 @@
 """bench.py -- MLPG frames/s on BASELINE.json configs[1] (batched MLPG, 256 utterances T~600,
 D=187 Merlin layout, 3 windows, per-frame diagonal variances, float32 in / float64 arithmetic).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One step = one pass of the hot path (banded W^T S^-1 W assemble + factor + solve for every static
 dimension of every utterance) over one batch of synthetic input.  Prints ONE JSON line (rank 0).
@@ -381,6 +381,18 @@ class Cfg5Pass(object):
         return worst
 
 
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, **arrays):
+    """--dump-outputs: each float32 / float64 array as out_dir/<name>.npy, DUMP_MAX_BYTES in all at most."""
+    assert all(a.dtype in (np.float32, np.float64) for a in arrays.values())
+    assert sum(a.nbytes for a in arrays.values()) <= DUMP_MAX_BYTES
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def _timed(fn, steps, warmup, barrier):
     import torch
     for _ in range(warmup):
@@ -580,6 +592,8 @@ def run_ours(args):
     kernel_ms = [a.elapsed_time(b) for a, b in kev]
     frames_all = float(n_rows)
     value = frames_all * args.steps / (total_ms * 1e-3)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, trajectories=d_out.cpu().numpy())
 
     # parity spot check of what was just timed (utterance 0, mgc stream) against the oracle
     parity = None
@@ -895,7 +909,12 @@ def main():
     ap.add_argument("--e2e-steps", type=int, default=20)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, save the trajectories of the last step as DIR/trajectories.npy "
+                         "(all utterances in batch order, (frames, 63) float32) for output-for-output comparison of builds")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.gpus != 1):
+        ap.error("--dump-outputs applies to the one-GPU run of --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

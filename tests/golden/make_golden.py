@@ -12,6 +12,7 @@ labelled ``restated`` in the file name.
 """
 import os
 import sys
+import types
 
 import numpy as np
 
@@ -182,7 +183,49 @@ def main():
             np.array(dist), np.array(path, dtype=np.int32), np.array(cells))
         d["c%d_exact_dist" % case], d["c%d_exact_path" % case] = np.array(de), np.array(pe, dtype=np.int32)
     np.savez_compressed(os.path.join(HERE, "dtw_restated_golden.npz"), **d)
+    reference_parity()
     print("wrote", os.listdir(HERE))
+
+
+def reference_parity():
+    """What tests/test_oracle_golden.py::test_oracle_vs_live_reference and
+    tests/test_host_logic_cpu.py::test_gmm_parameter_split_matches_reference compare against: the
+    reference's outputs on their inputs (same seeds and draw order), inputs stored beside them."""
+    oracle.import_reference()
+    from nnmnkwii import paramgen as G
+    from nnmnkwii.baseline.gmm import MLPGBase as RefMLPGBase
+    out = {}
+    rng = np.random.default_rng(7)
+    for wi, ws in enumerate(windows_set()):
+        for dt in (np.float32, np.float64):
+            for T in (3, 17, 64):
+                key = "live_w%d_%s_T%d" % (wi, np.dtype(dt).name, T)
+                D = 3 * len(ws)
+                m = rng.random((T, D)).astype(dt)
+                v = (rng.random((T, D)) + 0.01).astype(dt)
+                go = rng.standard_normal((T, 3)).astype(np.float32)
+                out[key + "_means"], out[key + "_vars"], out[key + "_go"] = m, v, go
+                out[key + "_y"] = G.mlpg(m, v, ws)
+                out[key + "_grad"] = G.mlpg_grad(m, v, ws, go)
+        out["live_w%d_R_T21" % wi] = G.unit_variance_mlpg_matrix(ws, 21)
+    # baseline.gmm.MLPGBase parameter split of a random full-covariance joint GMM (M=3, 2 x 4 dims)
+    gr = np.random.default_rng(0)
+    M, dim = 3, 4
+    A = gr.standard_normal((M, 2 * dim, 2 * dim))
+    cov = A @ A.transpose(0, 2, 1) + 0.5 * np.eye(2 * dim)
+    w = gr.random(M) + 0.1
+    gmm = types.SimpleNamespace(means_=gr.standard_normal((M, 2 * dim)), covariances_=cov, weights_=w / w.sum(),
+                                covariance_type="full")
+    out["split_means"], out["split_covars"], out["split_weights"] = gmm.means_, gmm.covariances_, gmm.weights_
+    for swap in (False, True):
+        for diff in (False, True):
+            ref = RefMLPGBase(gmm, swap=swap, diff=diff)
+            key = "split_swap%d_diff%d_" % (swap, diff)
+            for name in ("src_means", "tgt_means", "covarXX", "covarXY", "covarYX", "covarYY", "weights"):
+                out[key + name] = getattr(ref, name)
+            out[key + "num_mixtures"] = np.array(ref.num_mixtures)
+            out[key + "prec_chol"] = ref.px.precisions_cholesky_
+    np.savez_compressed(os.path.join(HERE, "reference_parity_golden.npz"), **out)
 
 
 if __name__ == "__main__":

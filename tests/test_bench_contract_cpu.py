@@ -43,3 +43,11 @@ def test_reference_arm_line_on_a_tiny_sample(monkeypatch):
     assert line["e2e"] == {"value": line["value"], "unit": "frames/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     cb = line["cpu_baseline"]
     assert cb["kind"] == ("reference" if oracle.reference_available() else "port") and cb["cores"] >= 1
+
+
+def test_dump_outputs_is_refused_where_it_does_not_apply(tmp_path):
+    for extra in (["--impl", "reference"], ["--gpus", "2"]):
+        cmd = [sys.executable, os.path.join(ROOT, "bench.py"), "--dump-outputs", str(tmp_path / "out")] + extra
+        out = subprocess.run(cmd, cwd=str(tmp_path), capture_output=True, text=True, timeout=600)
+        assert out.returncode == 2 and "--dump-outputs" in out.stderr
+    assert not (tmp_path / "out").exists()

@@ -1,11 +1,13 @@
 """Host-side logic that needs no GPU: stream layouts, the GMM parameter split of baseline.gmm
-(against the live reference when oracle/_ref is present), metric front-ends failing loudly."""
+(against the reference's stored outputs), metric front-ends failing loudly."""
+import os
 import types
 
 import numpy as np
 import pytest
 
 import oracle
+from conftest import ROOT
 
 
 def test_merlin_layout_chain_table():
@@ -32,17 +34,18 @@ def _random_gmm(seed=0, M=3, dim=4):
 
 @pytest.mark.parametrize("swap,diff", [(False, False), (True, False), (False, True), (True, True)])
 def test_gmm_parameter_split_matches_reference(swap, diff):
-    if not oracle.reference_available():
-        pytest.skip("oracle/_ref not built")
-    oracle.import_reference()
-    from nnmnkwii.baseline.gmm import MLPGBase as Ref
+    # the reference's MLPGBase attributes for _random_gmm(), stored by tests/golden/make_golden.py
     from nnmnkwii_b200.baseline.gmm import MLPG, MLPGBase
+    ref = np.load(os.path.join(ROOT, "tests", "golden", "reference_parity_golden.npz"))
     gmm = _random_gmm()
-    ours, ref = MLPGBase(gmm, swap=swap, diff=diff), Ref(gmm, swap=swap, diff=diff)
+    assert np.array_equal(gmm.means_, ref["split_means"]) and np.array_equal(gmm.covariances_, ref["split_covars"])
+    assert np.array_equal(gmm.weights_, ref["split_weights"])
+    ours = MLPGBase(gmm, swap=swap, diff=diff)
+    key = "split_swap%d_diff%d_" % (swap, diff)
     for name in ("src_means", "tgt_means", "covarXX", "covarXY", "covarYX", "covarYY", "weights"):
-        assert np.array_equal(getattr(ours, name), getattr(ref, name)), name
-    assert ours.num_mixtures == ref.num_mixtures
-    assert np.allclose(ours._prec_chol, ref.px.precisions_cholesky_, rtol=1e-12, atol=1e-14)
+        assert np.array_equal(getattr(ours, name), ref[key + name]), name
+    assert ours.num_mixtures == int(ref[key + "num_mixtures"])
+    assert np.allclose(ours._prec_chol, ref[key + "prec_chol"], rtol=1e-12, atol=1e-14)
     m = MLPG(gmm)  # default windows: static + delta (gmm.py:199-203)
     assert len(m.windows) == 2 and m.static_dim == 2
 

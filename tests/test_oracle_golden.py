@@ -1,11 +1,18 @@
 """CPU: pin the oracle (oracle/nnk_oracle.c) against the golden vectors generated from the
-UNMODIFIED reference (tests/golden/make_golden.py), against the reference's own known-answer
-tests, and - when oracle/_ref is present - against the reference itself."""
+UNMODIFIED reference (tests/golden/make_golden.py) and against the reference's own known-answer
+tests."""
+import os
+
 import numpy as np
 import pytest
 
 import oracle
-from conftest import rel_err, windows_set
+from conftest import ROOT, rel_err, windows_set
+
+
+@pytest.fixture(scope="module")
+def parity_golden():
+    return np.load(os.path.join(ROOT, "tests", "golden", "reference_parity_golden.npz"))
 
 
 def test_mlpg_oracle_matches_reference_golden(golden):
@@ -89,21 +96,18 @@ def test_mlpg_oracle_edge_cases():
         oracle.mlpg(m, v2, ws)
 
 
-@pytest.mark.skipif(not oracle.reference_available(), reason="oracle/_ref not built")
-def test_oracle_vs_live_reference():
-    oracle.import_reference()
-    from nnmnkwii import paramgen as G
-    rng = np.random.default_rng(7)
-    for ws in windows_set():
-        for dt in (np.float32, np.float64):
+def test_oracle_vs_live_reference(parity_golden):
+    # the reference's paramgen outputs on these inputs, stored by tests/golden/make_golden.py
+    for wi, ws in enumerate(windows_set()):
+        for dt in ("float32", "float64"):
             for T in (3, 17, 64):
-                D = 3 * len(ws)
-                m = rng.random((T, D)).astype(dt)
-                v = (rng.random((T, D)) + 0.01).astype(dt)
-                assert np.array_equal(G.mlpg(m, v, ws), oracle.mlpg(m, v, ws))
-                go = rng.standard_normal((T, 3)).astype(np.float32)
-                assert rel_err(oracle.mlpg_grad(m, v, ws, go), G.mlpg_grad(m, v, ws, go)) < 2e-6
-        assert np.abs(G.unit_variance_mlpg_matrix(ws, 21) - oracle.unit_variance_mlpg_matrix(ws, 21)).max() < 1e-7
+                key = "live_w%d_%s_T%d" % (wi, dt, T)
+                m, v, go = parity_golden[key + "_means"], parity_golden[key + "_vars"], parity_golden[key + "_go"]
+                assert m.dtype == dt and m.shape == (T, 3 * len(ws))
+                assert np.array_equal(parity_golden[key + "_y"], oracle.mlpg(m, v, ws)), key
+                assert rel_err(oracle.mlpg_grad(m, v, ws, go), parity_golden[key + "_grad"]) < 2e-6, key
+        R = parity_golden["live_w%d_R_T21" % wi]
+        assert np.abs(R - oracle.unit_variance_mlpg_matrix(ws, 21)).max() < 1e-7
 
 
 def test_delta_features_oracle(golden):
